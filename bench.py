@@ -3,7 +3,7 @@
 
 Metric (BASELINE.json): GAE forward+backward trajectory-steps/s at 1/2/4/8 B200, plus % of the HBM roofline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one GAE forward + one GAE adjoint over one batch of synthetic trajectories (T=1024, B=65536 per GPU,
@@ -27,6 +27,10 @@ shard (global batch N*65536, no data-path collective => weak scaling).
 
 `--impl reference` times the CPU implementation (the oracle port: the reference's own CPU path is the Python/PyTorch
 `hpc_rll.origin`, which does not exist on the GPU box) on the same config.
+
+`--dump-outputs DIR` writes what the last timed step returned to its caller (adv, grad_value, grad_reward) as
+DIR/<name>.npy, float32, restricted to a fixed seeded sample of columns (at most 16 MB per output).  The inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -295,6 +299,22 @@ def ops_block(torch, peak):
     return out
 
 
+def dump_outputs(out_dir, outputs, B, suffix=""):
+    """Write the last timed step's outputs as out_dir/<name><suffix>.npy (float32).  Every output is (rows, B); a full
+    one is 268 MB at the default size, so a fixed sample of whole columns (complete trajectories) is kept: the same
+    seeded choice of columns in every output and every run, at most 2^22 elements (16 MB) per output."""
+    import numpy as np
+    import torch
+    rows = max(t.shape[0] for t in outputs.values())
+    ncols = min(B, max(1, (1 << 22) // rows))
+    cols = np.sort(np.random.default_rng(0).choice(B, size=ncols, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        idx = torch.from_numpy(cols).to(t.device)
+        a = t.detach().index_select(1, idx).float().cpu().numpy()
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
+
+
 def run_ours(args):
     import torch
     from di_hpc_b200 import _abi
@@ -324,9 +344,10 @@ def run_ours(args):
     gadv = torch.randn(T, B, device=dev, generator=gen)
     gae = GAE(T, B)
 
-    def step():  # the API north_star names: module forward + autograd backward
+    def step():  # the API north_star names: module forward + autograd backward -> what its caller receives
         adv = gae(value, reward, GAMMA, LAMBDA)
-        return torch.autograd.grad(adv, [value, reward], grad_outputs=gadv)
+        grad_value, grad_reward = torch.autograd.grad(adv, [value, reward], grad_outputs=gadv)
+        return {"adv": adv, "grad_value": grad_value, "grad_reward": grad_reward}
 
     def barrier():
         if dist is not None:
@@ -342,20 +363,25 @@ def run_ours(args):
     sampler = ClockSampler(local) if rank == 0 else None
     if sampler:
         sampler.start()
+    # each step's outputs are held until the next step returns, in warm-up as in the timed loop, so that the
+    # allocator already holds both sets of output buffers when the timing starts
     for _ in range(W):
-        step()
+        last = step()
     # ---- timed region: exactly K steps ------------------------------------------------------
     barrier()
     n0 = _abi.launch_count()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(K):
-        step()
+        last = step()
     e1.record()
     barrier()
     launches = _abi.launch_count() - n0
     ms_per_step = max_over_ranks(e0.elapsed_time(e1)) / K
     value_metric = T * B * world / (ms_per_step * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last, B, "" if world == 1 else "_rank%d" % rank)
+    del last
 
     # ---- the same step per call (synchronise after each) and through the raw C ABI (no autograd, no allocation) ----
     per_call = []
@@ -625,7 +651,14 @@ def main():
     ap.add_argument("--T", type=int, default=T_DEFAULT)
     ap.add_argument("--B", type=int, default=B_DEFAULT, help="columns per GPU")
     ap.add_argument("--no-extras", action="store_true", help="skip the ops / c4 / loss_allreduce blocks")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs (adv, grad_value, grad_reward; a fixed sample of columns) "
+                         "as DIR/<name>.npy; the inputs are seeded, so runs with the same arguments are comparable")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     global OUT
     OUT = _claim_stdout()
     if args.impl == "reference":

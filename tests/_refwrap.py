@@ -1,31 +1,42 @@
-"""Load the UNMODIFIED reference wrappers (hpc_rll/rl_utils/*.py of DI-hpc) under alias module names, with
-`import hpc_rl_utils` inside them resolving to this repo's shim (hpc_rl_utils/__init__.py -> csrc_torch/legacy.cpp).
-Sources: /root/reference (build container) or baseline/_ref/ref_wrappers (staged by tools/stage_ref_wrappers.sh; the
-only copy that exists on the GPU box).  Never the product's own hpc_rll package."""
-import importlib.util
+"""The UNMODIFIED reference wrappers (hpc_rll/rl_utils/*.py of DI-hpc) as recorded calls into their native module.
+
+Those wrappers own no arithmetic: each module registers scratch buffers and each autograd Function hands
+(input list, output list, scalars) to one `hpc_rl_utils` binding and returns some of the buffers.
+tests/golden/ref_wrapper_calls.json (written by tests/golden/make_wrapper_trace.py from the reference) records,
+per scenario, every such call, the shape / dtype / initial fill of every buffer, and which binding output the
+user receives.  `replay` issues exactly those calls against this repository's `hpc_rl_utils` shim, which is what
+a DI-hpc user gets by swapping the extension under the unmodified wrappers."""
+import json
 import os
-import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CANDIDATES = [os.path.join(ROOT, "baseline", "_ref", "ref_wrappers"), "/root/reference/hpc_rll/rl_utils"]
+TRACE_PATH = os.path.join(ROOT, "tests", "golden", "ref_wrapper_calls.json")
+
+with open(TRACE_PATH) as _f:
+    TRACE = json.load(_f)
 
 
-def wrapper_dir():
-    for d in CANDIDATES:
-        if os.path.exists(os.path.join(d, "vtrace.py")):
-            return d
-    return None
+def scenario(name):
+    return TRACE["scenarios"][name]
 
 
-def load(name):
-    d = wrapper_dir()
-    if d is None:
-        return None
-    alias = "ref_wrapper_" + name
-    if alias in sys.modules:
-        return sys.modules[alias]
-    spec = importlib.util.spec_from_file_location(alias, os.path.join(d, name + ".py"))
-    mod = importlib.util.module_from_spec(spec)
-    sys.modules[alias] = mod
-    spec.loader.exec_module(mod)
-    return mod
+def replay(name, inputs, native, device="cuda"):
+    """Issue the recorded calls of scenario `name` on `native` (the `hpc_rl_utils` module) with `inputs`
+    (dict of tensors named as recorded) -> dict result name -> the binding output the wrapper returns."""
+    import torch
+    sc = scenario(name)
+    for k, spec in sc["inputs"].items():
+        t = inputs[k]
+        assert list(t.shape) == spec["shape"] and str(t.dtype) == "torch." + spec["dtype"], (name, k, t.shape, t.dtype)
+    bufs = {int(k): torch.full(b["shape"], b["fill"], dtype=getattr(torch, b["dtype"]), device=device)
+            for k, b in sc["buffers"].items()}
+
+    def get(ref):
+        return inputs[ref["input"]] if "input" in ref else bufs[ref["buffer"]]
+
+    outs = []
+    for c in sc["calls"]:
+        o = [get(r) for r in c["outputs"]]
+        getattr(native, c["fn"])([get(r) for r in c["inputs"]], o, *c["scalars"])
+        outs.append(o)
+    return {k: outs[c][i] for k, (c, i) in sc["results"].items()}

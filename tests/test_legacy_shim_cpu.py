@@ -1,7 +1,8 @@
 """The native boundary of the reference: a module importable as `hpc_rl_utils` exporting the 30 binding names of
-/root/reference/src/rl_utils/entry.cpp:9-38 with tensor-list signatures.  CPU part: names, arities, and that the
-UNMODIFIED reference wrappers import and construct against the shim (no kernel runs without a GPU)."""
-import re
+DI-hpc's src/rl_utils/entry.cpp:9-38 with tensor-list signatures.  CPU part: names, arities, and that every call the
+UNMODIFIED reference wrappers make (recorded in tests/golden/ref_wrapper_calls.json) reaches a shim binding that takes
+those arguments (no kernel runs without a GPU)."""
+import os
 
 import pytest
 
@@ -27,25 +28,19 @@ def test_all_reference_binding_names_exist_with_reference_arity():
 
 
 def test_entry_cpp_lists_exactly_these_names():
-    import os
-    p = "/root/reference/src/rl_utils/entry.cpp"
-    if not os.path.exists(p):
-        pytest.skip("reference tree not present")
-    names = re.findall(r'm\.def\("(\w+)"', open(p).read())
-    assert sorted(names) == sorted(list(HOT) + PAD)
+    assert sorted(_refwrap.TRACE["entry_cpp_bindings"]) == sorted(list(HOT) + PAD)
 
 
 @pytest.mark.parametrize("mod", ["gae", "td", "upgo", "vtrace", "ppo"])
 def test_unmodified_reference_wrappers_bind_to_the_shim(mod):
-    if _refwrap.wrapper_dir() is None:
-        pytest.skip("reference wrappers not available (run tools/stage_ref_wrappers.sh in the build container)")
     import hpc_rl_utils
-    m = _refwrap.load(mod)
-    assert m.hpc_rl_utils is hpc_rl_utils
-    used = set(re.findall(r"hpc_rl_utils\.(\w+)", open(m.__file__).read()))
+    # `import hpc_rl_utils` inside the wrappers resolves to this repository's shim
+    assert os.path.dirname(os.path.abspath(hpc_rl_utils.__file__)) == os.path.join(_refwrap.ROOT, "hpc_rl_utils")
+    used = _refwrap.TRACE["wrapper_uses"][mod]
     assert used and all(hasattr(hpc_rl_utils, u) for u in used), used
-    # the modules build their scratch buffers on the CPU just like in the reference
-    ctor = {"gae": lambda: m.GAE(4, 3), "td": lambda: (m.TDLambda(4, 3), m.QNStepTD(4, 3, 2), m.DistNStepTD(4, 3, 2, 5),
-                                                      m.QRDQNNStepTDError(8, 4, 3, 2), m.IQNNStepTDError(8, 9, 4, 3, 2)),
-            "upgo": lambda: m.UPGO(4, 3, 2), "vtrace": lambda: m.VTrace(4, 3, 2), "ppo": lambda: m.PPO(3, 2)}
-    ctor[mod]()
+    # every recorded call of this wrapper: (inputs, outputs, scalars...) matches the binding's arity
+    calls = [c for s in _refwrap.TRACE["scenarios"].values() if s["module"] == mod for c in s["calls"]]
+    assert calls and {c["fn"] for c in calls} <= set(used)
+    for c in calls:
+        sig = getattr(hpc_rl_utils, c["fn"]).__doc__.splitlines()[0]
+        assert sig.count("arg") == 2 + len(c["scalars"]), (c["fn"], sig, c["scalars"])

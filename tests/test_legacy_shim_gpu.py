@@ -3,8 +3,9 @@
 (a) `test_names_*`: each of the 19 hot-path `hpc_rl_utils` names called directly with tensor lists in the reference
     launchers' positional order (src/rl_utils/*.cu `index++`; buffers shaped as the reference modules register them),
     results compared with the oracle.
-(b) `test_reference_wrappers_*`: the UNMODIFIED reference wrappers (staged copy of hpc_rll/rl_utils/*.py) running on the
-    shim, forward + autograd backward, compared with the oracle -- what a DI-hpc user gets by swapping the extension.
+(b) `test_reference_wrappers_*`: the calls the UNMODIFIED reference wrappers (hpc_rll/rl_utils/*.py) make into their
+    native module in forward + autograd backward (recorded in tests/golden/ref_wrapper_calls.json), issued on the shim
+    and compared with the oracle -- what a DI-hpc user gets by swapping the extension.
 """
 import numpy as np
 import pytest
@@ -187,26 +188,23 @@ def test_names_upgo_vtrace_ppo():
 
 
 # ------------------------------------------------------------------------------------------------ (b) reference wrappers
-def _ref(mod):
+def _replay(name, **inputs):
+    """the calls the unmodified reference wrapper makes in scenario `name`, issued on the shim (tests/_refwrap.py)"""
     need_cuda()
-    m = _refwrap.load(mod)
-    if m is None:
-        pytest.skip("reference wrappers not staged (tools/stage_ref_wrappers.sh)")
-    return m
+    import hpc_rl_utils
+    return _refwrap.replay(name, inputs, hpc_rl_utils)
 
 
 def test_reference_wrappers_gae_tdlambda():
     g = rng(11)
     T, B = 1024, 64  # tests/test_gae.py:10-11, tests/test_tdlambda.py:10-11
     value, reward, weight = scan_inputs(g, T, B)
-    adv = _ref("gae").GAE(T, B).cuda()(dev(value), dev(reward))
+    adv = _replay("gae", value=dev(value), reward=dev(reward))["adv"]
     close(host(adv), orc.gae_forward(value, reward, np.float32(0.99), np.float32(0.97)), "adv")
-    v = dev(value).requires_grad_(True)
-    loss = _ref("td").TDLambda(T, B).cuda()(v, dev(reward), dev(weight))
-    loss.backward()
+    r = _replay("td_lambda", value=dev(value), reward=dev(reward), weight=dev(weight))
     o = orc.td_lambda(value, reward, weight, np.float32(0.9), np.float32(0.8))
-    close(float(loss.item()), o["loss"], "loss")
-    close(host(v.grad) * T * B, o["grad_value"] * T * B, "grad_value")
+    close(float(r["loss"].item()), o["loss"], "loss")
+    close(host(r["grad_value"]) * T * B, o["grad_value"] * T * B, "grad_value")
 
 
 def test_reference_wrappers_vtrace_upgo_ppo():
@@ -216,85 +214,70 @@ def test_reference_wrappers_vtrace_upgo_ppo():
     tgt = (g.standard_normal((T, B, N)) * 1.5).astype(np.float32)
     beh = (g.standard_normal((T, B, N)) * 1.5).astype(np.float32)
     act = g.integers(0, N, (T, B)).astype(np.int64)
-    t, v = dev(tgt).requires_grad_(True), dev(value).requires_grad_(True)
-    l = _ref("vtrace").VTrace(T, B, N).cuda()(t, dev(beh), dev(act), v, dev(reward))  # weight None -> module ones
+    # weight None -> module ones; upstream gradients 1, 0.5, -0.25 of the three losses
+    r = _replay("vtrace", target_output=dev(tgt), behaviour_output=dev(beh), action=dev(act), value=dev(value),
+                reward=dev(reward))
     coef = [1.0, 0.5, -0.25]
-    (coef[0] * l.policy_loss + coef[1] * l.value_loss + coef[2] * l.entropy_loss).sum().backward()
     o = orc.vtrace(tgt, beh, act, value, reward, None, coef=coef)
-    for got, nm in zip(l, ("policy_loss", "value_loss", "entropy_loss")):
-        close(float(got.item()), o[nm], nm)
-    close(host(t.grad) * T * B, o["grad_target_output"] * T * B, "vtrace grad_target_output")
-    close(host(v.grad) * T * B, o["grad_value"] * T * B, "vtrace grad_value")
+    for nm in ("policy_loss", "value_loss", "entropy_loss"):
+        close(float(r[nm].item()), o[nm], nm)
+    close(host(r["grad_target_output"]) * T * B, o["grad_target_output"] * T * B, "vtrace grad_target_output")
+    close(host(r["grad_value"]) * T * B, o["grad_value"] * T * B, "vtrace grad_value")
     rhos = (g.random((T, B)) * 2).astype(np.float32)
-    t2 = dev(tgt).requires_grad_(True)
-    loss = _ref("upgo").UPGO(T, B, N).cuda()(t2, dev(rhos), dev(act), dev(reward), dev(value))
-    loss.sum().backward()
+    r = _replay("upgo", target_output=dev(tgt), rhos=dev(rhos), action=dev(act), reward=dev(reward), value=dev(value))
     o = orc.upgo(tgt, rhos, act, reward, value)
-    close(float(loss.item()), o["loss"], "upgo loss")
-    close(host(t2.grad) * T * B, o["grad_target_output"] * T * B, "upgo grad")
+    close(float(r["loss"].item()), o["loss"], "upgo loss")
+    close(host(r["grad_target_output"]) * T * B, o["grad_target_output"] * T * B, "upgo grad")
     Bp = 128  # tests/test_ppo.py:11-12
     lo = g.standard_normal((Bp, N)).astype(np.float32)
     ln = (lo + 0.3 * g.standard_normal((Bp, N))).astype(np.float32)
     a = g.integers(0, N, (Bp, )).astype(np.int64)
     vn, vo, adv, ret = (g.standard_normal(Bp).astype(np.float32) for _ in range(4))
-    lnt, vnt = dev(ln).requires_grad_(True), dev(vn).requires_grad_(True)
-    loss, info = _ref("ppo").PPO(Bp, N).cuda()(lnt, dev(lo), dev(a), vnt, dev(vo), dev(adv), dev(ret), None, 0.2, True, None)
-    (loss.policy_loss + 0.5 * loss.value_loss - 0.01 * loss.entropy_loss).sum().backward()
+    # weight None, clip 0.2, value clip on, dual clip None; loss = policy + 0.5 value - 0.01 entropy
+    r = _replay("ppo", logits_new=dev(ln), logits_old=dev(lo), action=dev(a), value_new=dev(vn), value_old=dev(vo),
+                adv=dev(adv), **{"return": dev(ret)})
     o = orc.ppo(ln, lo, a, vn, vo, adv, ret, None, 0.2, True, None, [1.0, 0.5, -0.01])
-    for got, nm in zip(loss, ("policy_loss", "value_loss", "entropy_loss")):
-        close(float(got.item()), o[nm], "ppo " + nm)
-    close(info.approx_kl, o["approx_kl"], "approx_kl")
-    close(host(lnt.grad) * Bp, o["grad_logits_new"] * Bp, "ppo grad_logits_new")
-    close(host(vnt.grad) * Bp, o["grad_value_new"] * Bp, "ppo grad_value_new")
+    for nm in ("policy_loss", "value_loss", "entropy_loss"):
+        close(float(r[nm].item()), o[nm], "ppo " + nm)
+    close(float(r["approx_kl"].item()), o["approx_kl"], "approx_kl")
+    close(host(r["grad_logits_new"]) * Bp, o["grad_logits_new"] * Bp, "ppo grad_logits_new")
+    close(host(r["grad_value_new"]) * Bp, o["grad_value_new"] * Bp, "ppo grad_value_new")
 
 
 def test_reference_wrappers_nstep_family():
     g = rng(13)
-    td = _ref("td")
     T, B, N = 10, 89, 7
     inp = nstep_inputs(g, T, B, N)
     dv = {k: dev(v) for k, v in inp.items()}
-    for rescale, cls in ((False, td.QNStepTD), (True, td.QNStepTDRescale)):
+    for rescale, name in ((False, "q_nstep_td"), (True, "q_nstep_td_rescale")):  # gamma 0.95
         q, nq = g.standard_normal((B, N), dtype=np.float32), g.standard_normal((B, N), dtype=np.float32)
-        qt = dev(q).requires_grad_(True)
-        loss, tde = cls(T, B, N).cuda()(qt, dev(nq), dv["action"], dv["next_n_action"], dv["reward"], dv["done"],
-                                        dv["weight"], 0.95)
-        loss.sum().backward()
+        r = _replay(name, q=dev(q), next_n_q=dev(nq), **dv)
         o = orc.q_nstep_td(q, nq, inp["action"], inp["next_n_action"], inp["reward"], inp["done"], inp["weight"],
                            np.float32(0.95), rescale)
-        close(float(loss.item()), o["loss"], "q loss")
-        close(host(tde), o["td_error_per_sample"], "q td")
-        close(host(qt.grad) * B, o["grad_q"] * B, "grad_q")
+        close(float(r["loss"].item()), o["loss"], "q loss")
+        close(host(r["td_error_per_sample"]), o["td_error_per_sample"], "q td")
+        close(host(r["grad_q"]) * B, o["grad_q"] * B, "grad_q")
     A = 51
     sm = lambda x: (np.exp(x) / np.exp(x).sum(-1, keepdims=True)).astype(np.float32)  # noqa: E731
     dist, ndist = sm(g.standard_normal((B, N, A))), sm(g.standard_normal((B, N, A)))
-    dt = dev(dist).requires_grad_(True)
-    loss, tde = td.DistNStepTD(T, B, N, A).cuda()(dt, dev(ndist), dv["action"], dv["next_n_action"], dv["reward"],
-                                                  dv["done"], dv["weight"], 0.95, -10.0, 10.0)
-    loss.sum().backward()
+    r = _replay("dist_nstep_td", q=dev(dist), next_n_q=dev(ndist), **dv)  # gamma 0.95, support [-10, 10]
     o = orc.dist_nstep_td(dist, ndist, inp["action"], inp["next_n_action"], inp["reward"], inp["done"], inp["weight"],
                           np.float32(0.95), -10.0, 10.0)
-    close(float(loss.item()), o["loss"], "dist loss")
-    close(host(dt.grad) * B, o["grad_dist"] * B, "grad_dist")
+    close(float(r["loss"].item()), o["loss"], "dist loss")
+    close(host(r["grad_q"]) * B, o["grad_dist"] * B, "grad_dist")
     tau, tau_p = 39, 34  # tests/test_qrdqn_nstep_td_error.py:10-14
     q, nq = g.standard_normal((B, N, tau), dtype=np.float32), g.standard_normal((B, N, tau), dtype=np.float32)
-    qt = dev(q).requires_grad_(True)
-    loss, tde = td.QRDQNNStepTDError(tau, T, B, N).cuda()(qt, dev(nq), dv["action"], dv["next_n_action"], dv["reward"],
-                                                          dv["done"], 0.95, dv["weight"])
-    loss.sum().backward()
+    r = _replay("qrdqn_nstep_td", q=dev(q), next_n_q=dev(nq), **dv)  # gamma 0.95, value_gamma None
     o = orc.qrdqn_nstep_td(q, nq, inp["action"], inp["next_n_action"], inp["reward"], inp["done"], inp["weight"], None,
                            np.float32(0.95))
-    close(float(loss.item()), o["loss"], "qrdqn loss")
-    close(host(tde), o["td_error_per_sample"], "qrdqn td")
-    close(host(qt.grad) * B, o["grad_q"] * B, "qrdqn grad_q")
+    close(float(r["loss"].item()), o["loss"], "qrdqn loss")
+    close(host(r["td_error_per_sample"]), o["td_error_per_sample"], "qrdqn td")
+    close(host(r["grad_q"]) * B, o["grad_q"] * B, "qrdqn grad_q")
     qi, nqi = g.standard_normal((tau, B, N), dtype=np.float32), g.standard_normal((tau_p, B, N), dtype=np.float32)
     rq = g.random((tau, B)).astype(np.float32)
-    qit = dev(qi).requires_grad_(True)
-    loss, tde = td.IQNNStepTDError(tau, tau_p, T, B, N).cuda()(qit, dev(nqi), dv["action"], dv["next_n_action"],
-                                                               dv["reward"], dv["done"], dev(rq), 0.95, 0.9, dv["weight"])
-    loss.sum().backward()
+    r = _replay("iqn_nstep_td", q=dev(qi), next_n_q=dev(nqi), replay_quantiles=dev(rq), **dv)  # gamma 0.95, kappa 0.9
     o = orc.iqn_nstep_td(qi, nqi, inp["action"], inp["next_n_action"], inp["reward"], inp["done"], rq, inp["weight"], None,
                          np.float32(0.95), np.float32(0.9))
-    close(float(loss.item()), o["loss"], "iqn loss")
-    close(host(tde), o["td_error_per_sample"], "iqn td")
-    close(host(qit.grad) * B, o["grad_q"] * B, "iqn grad_q")
+    close(float(r["loss"].item()), o["loss"], "iqn loss")
+    close(host(r["td_error_per_sample"]), o["td_error_per_sample"], "iqn td")
+    close(host(r["grad_q"]) * B, o["grad_q"] * B, "iqn grad_q")

@@ -2,7 +2,6 @@
 TMA tensor loads AND stores in the headline GAE kernels, bulk copies where the docs say so, packed fp32 in the pairwise
 quantile sweep -- and no floating-point atomic anywhere (every reduction has a fixed order)."""
 import os
-import shutil
 import sys
 
 import pytest
@@ -13,10 +12,10 @@ sys.path.insert(0, ROOT)
 
 @pytest.fixture(scope="module")
 def sass():
-    if shutil.which("cuobjdump") is None:
-        pytest.skip("cuobjdump not on PATH")
     from di_hpc_b200 import build
     from tools import sass_opcodes
+    if sass_opcodes.cuobjdump() is None:
+        pytest.skip("cuobjdump not found (neither on PATH nor in the CUDA toolkit)")
     lib = build.build()
     kernels, atomics, arch = sass_opcodes.parse(lib)
     assert len(kernels) > 100
