@@ -68,10 +68,12 @@ SIGNATURES = {
     "hpc_rll_unpad_batch": (c_int, [c_vp] * 4 + [c_i64, c_vp]),
     "hpc_rll_oracle_split_group": (c_int, [c_vp, c_i64, c_int, c_int, c_vp]),
     "hpc_rll_sample_split_group": (c_int, [c_vp, c_i64, c_int, c_int, ctypes.c_uint64, c_vp, c_vp]),
+    "hpc_rll_scatter_connection_forward": (c_int, [c_vp] * 3 + [c_i64] * 5 + [c_int, c_vp]),
+    "hpc_rll_scatter_connection_backward": (c_int, [c_vp] * 3 + [c_i64] * 5 + [c_vp]),
 }
 
 OP_GAE, OP_TD_LAMBDA, OP_VTRACE, OP_UPGO, OP_PPO, OP_Q_NSTEP_TD, OP_DIST_NSTEP_TD, OP_QRDQN_NSTEP_TD, \
-    OP_IQN_NSTEP_TD, OP_GAE_MOMENTS = range(10)
+    OP_IQN_NSTEP_TD, OP_GAE_MOMENTS, OP_SCATTER_CONNECTION = range(11)
 
 _lib = None
 

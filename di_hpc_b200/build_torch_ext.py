@@ -3,7 +3,9 @@ It contains no kernels and links against libhpc_rll_b200.so (rpath $ORIGIN):
   ext.cpp       list-of-tensor host work of the padding ops + the reference's 11 padding binding names
   fast_ops.cpp  C++ ``torch::autograd::Function`` per op -- what the nn.Modules of hpc_rll.rl_utils call
   legacy.cpp    the reference's 19 hot-path ``hpc_rl_utils`` binding names (tensor-list signatures)
-The top-level package ``hpc_rl_utils`` re-exports this module under the reference's name.
+  network.cpp   the reference's ``hpc_torch_utils_network`` ScatterConnection names, in the submodule ``_network``
+The top-level packages ``hpc_rl_utils`` and ``hpc_torch_utils_network`` re-export this module (and its ``_network``
+submodule) under the reference's names.
 
     python -m di_hpc_b200.build_torch_ext
 """
@@ -15,7 +17,7 @@ import sysconfig
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SRC_DIR = os.path.join(HERE, "csrc_torch")
-SRCS = [os.path.join(SRC_DIR, f) for f in ("ext.cpp", "fast_ops.cpp", "legacy.cpp")]
+SRCS = [os.path.join(SRC_DIR, f) for f in ("ext.cpp", "fast_ops.cpp", "legacy.cpp", "network.cpp")]
 OBJ_DIR = os.path.join(HERE, "_lib", "obj")
 OUT_DIR = os.path.join(HERE, "_lib")
 NAME = "hpc_rl_utils_b200"

@@ -40,7 +40,7 @@ int sm_count() {
 static void init_cfg() {
     static const char* names[HPC_RLL_OP_COUNT] = {"GAE", "TD_LAMBDA", "VTRACE", "UPGO", "PPO",
                                                   "Q_NSTEP_TD", "DIST_NSTEP_TD", "QRDQN_NSTEP_TD", "IQN_NSTEP_TD",
-                                                  "GAE_MOMENTS"};
+                                                  "GAE_MOMENTS", "SCATTER_CONNECTION"};
     for (int i = 0; i < HPC_RLL_OP_COUNT; ++i) {
         char key[64];
         snprintf(key, sizeof(key), "HPC_RLL_CFG_%s", names[i]);

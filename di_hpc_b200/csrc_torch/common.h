@@ -1,5 +1,6 @@
 // common.h -- helpers shared by the torch/pybind layer (ext.cpp: padding lists; fast_ops.cpp: C++ autograd
-// functions behind hpc_rll.rl_utils; legacy.cpp: the reference's 19 `hpc_rl_utils` tensor-list entry points).
+// functions behind hpc_rll.rl_utils and hpc_rll.torch_utils.network; legacy.cpp: the reference's 19 `hpc_rl_utils`
+// tensor-list entry points; network.cpp: the reference's `hpc_torch_utils_network` ScatterConnection entry points).
 // Nothing here computes: every function ends in a call into the C ABI (include/hpc_rll_b200.h).
 #pragma once
 #include <c10/cuda/CUDAGuard.h>
@@ -46,5 +47,7 @@ inline Tensor gscalar(const Tensor& g, const Tensor& like) {
 
 void register_fast_ops(pybind11::module& m);
 void register_legacy(pybind11::module& m);
+void register_fast_network_ops(pybind11::module& net);
+void register_network_legacy(pybind11::module& net);
 
 }  // namespace hpcrl

@@ -223,6 +223,10 @@ py::list group_pad_nd(const std::vector<torch::Tensor>& inputs, int ndim, int gr
 PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
     hpcrl::register_fast_ops(m);  // C++ autograd functions behind hpc_rll.rl_utils (fast_ops.cpp)
     hpcrl::register_legacy(m);    // the reference's 19 hot-path `hpc_rl_utils` names (legacy.cpp)
+    // hpc_rll.torch_utils.network: its autograd op and the reference's `hpc_torch_utils_network` names
+    pybind11::module net = m.def_submodule("_network", "ScatterConnection (hpc_rll.torch_utils.network)");
+    hpcrl::register_fast_network_ops(net);  // fast_ops.cpp
+    hpcrl::register_network_legacy(net);    // network.cpp
     m.def("pad_nd", &pad_nd, "pad a list of n-D tensors: (new_x, mask, flat shapes)");
     m.def("group_pad_nd", &group_pad_nd, "sort + split + pad in one call");
     m.def("unpad_nd", [](const torch::Tensor& x, const std::vector<int>& s, int ndim) { return unpad_forward(x, s, ndim); },

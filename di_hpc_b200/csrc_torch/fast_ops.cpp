@@ -430,7 +430,50 @@ struct P2PAllReduceFn : public Function<P2PAllReduceFn> {
     }
 };
 
+// ------------------------------------------------------------------------------------------------ ScatterConnection
+// x (B,M,N) fp32, location (B,M,2) int64 (y, x) -> out (B,N,H,W), always a fresh tensor; backward needs only location
+struct ScatterConnectionFn : public Function<ScatterConnectionFn> {
+    static Tensor forward(AutogradContext* ctx, const Tensor& x_, const Tensor& location_, int64_t H, int64_t W,
+                          int64_t mode) {
+        const Tensor x = f32(x_, "x"), loc = i64(location_, "location");
+        TORCH_CHECK_VALUE(x.dim() == 3, "x must be (B, M, N), got ", x.sizes());
+        const int64_t B = x.size(0), M = x.size(1), N = x.size(2);
+        TORCH_CHECK_VALUE(loc.dim() == 3 && loc.size(0) == B && loc.size(1) == M && loc.size(2) == 2,
+                          "location must be (B, M, 2)=(", B, ", ", M, ", 2), got ", loc.sizes());
+        TORCH_CHECK(loc.device() == x.device(), "x and location must live on one CUDA device");
+        TORCH_CHECK_VALUE(H >= 0 && W >= 0, "H and W must be non-negative");
+        c10::cuda::CUDAGuard guard(x.device());
+        Tensor out = torch::empty({B, N, H, W}, x.options());
+        ck(hpc_rll_scatter_connection_forward(fp(x), ip(loc), fpm(out), B, M, N, H, W, static_cast<int>(mode),
+                                              cur_stream()),
+           "hpc_rll_scatter_connection_forward");
+        ctx->save_for_backward({loc});
+        ctx->saved_data["N"] = N;
+        return out;
+    }
+    static variable_list backward(AutogradContext* ctx, variable_list grads) {
+        const Tensor loc = ctx->get_saved_variables()[0];
+        const Tensor g = f32(grads[0], "grad_out");
+        const int64_t B = loc.size(0), M = loc.size(1), N = ctx->saved_data["N"].toInt(), H = g.size(2), W = g.size(3);
+        c10::cuda::CUDAGuard guard(g.device());
+        Tensor gx = torch::empty({B, M, N}, g.options());
+        ck(hpc_rll_scatter_connection_backward(fp(g), ip(loc), fpm(gx), B, M, N, H, W, cur_stream()),
+           "hpc_rll_scatter_connection_backward");
+        return {gx, Tensor(), Tensor(), Tensor(), Tensor()};
+    }
+};
+
 }  // namespace
+
+// the ops of hpc_rll.torch_utils.network, in the extension's `_network` submodule (keeps the names of the top-level
+// module -- what `hpc_rl_utils` re-exports -- exactly the reference's rl_utils set plus the rl_utils fast ops)
+void register_fast_network_ops(pybind11::module& net) {
+    net.def("scatter_connection",
+            [](const Tensor& x, const Tensor& loc, int64_t H, int64_t W, int64_t mode) {
+                return ScatterConnectionFn::apply(x, loc, H, W, mode);
+            },
+            "ScatterConnection forward (mode 0 cover, 1 add) with autograd -- C++ twin of ScatterConnectionFunction");
+}
 
 void register_fast_ops(pybind11::module& m) {
     m.def("allreduce_scalars_p2p",

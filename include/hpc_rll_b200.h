@@ -47,7 +47,8 @@ extern "C" {
 #define HPC_RLL_OP_QRDQN_NSTEP_TD 7
 #define HPC_RLL_OP_IQN_NSTEP_TD 8
 #define HPC_RLL_OP_GAE_MOMENTS 9 /* workspace sizing only; tuning follows HPC_RLL_OP_GAE */
-#define HPC_RLL_OP_COUNT 10
+#define HPC_RLL_OP_SCATTER_CONNECTION 10 /* no workspace; tuning: bit 0 forward thread stores, bit 1 backward gather */
+#define HPC_RLL_OP_COUNT 11
 
 /* ---- library ------------------------------------------------------------------------------ */
 const char* hpc_rll_version(void);
@@ -300,6 +301,23 @@ int hpc_rll_unpad_batch(const float* const* src, float* const* dst, const int32_
 int hpc_rll_oracle_split_group(const int64_t* shapes, int64_t n, int ndim, int group, int64_t* positions);
 int hpc_rll_sample_split_group(const int64_t* shapes, int64_t n, int ndim, int group, uint64_t seed,
                                int64_t* starts, int* n_groups);
+
+/* ---- ScatterConnection (AlphaStar-style entity -> spatial map scatter) ----------------------------
+ * replaces ScatterConnectionForward / ScatterConnectionBackward of the reference's `hpc_torch_utils_network`
+ * (/root/reference/src/torch_utils/network/scatter_connection.cu:8-76, kernels
+ * include/hpc/rll/cuda/torch_utils/network/scatter_connection_kernel.h:60-120); semantics of
+ * hpc_rll/origin/scatter_connection.py:25-64 on the CPU, i.e. sequential in entity order m.
+ *   forward : x (B,M,N), location (B,M,2) int64 pairs (y, x) -> out (B,N,H,W), every element written once:
+ *             mode 1 (add)   out[b,n,y*W+x] = ((0.f + x[b,m0,n]) + x[b,m1,n]) + ... in ascending m
+ *             mode 0 (cover) out[b,n,y*W+x] = x[b,m_last,n] (the last entity at a cell wins)
+ *             cells no entity lands on are +0.f; no memset is needed before the call
+ *   backward: grad_out (B,N,H,W) -> grad_x (B,M,N), grad_x[b,m,n] = grad_out[b,n,y*W+x] (both modes)
+ * An entity with y outside [0,H) or x outside [0,W) writes nothing and gets a zero gradient.  No atomics:
+ * results are bit-identical run to run.  No workspace.  Contiguous tensors; any 4-byte alignment. */
+int hpc_rll_scatter_connection_forward(const float* x, const int64_t* location, float* out, int64_t B, int64_t M,
+                                       int64_t N, int64_t H, int64_t W, int mode /* 0 cover, 1 add */, void* stream);
+int hpc_rll_scatter_connection_backward(const float* grad_out, const int64_t* location, float* grad_x, int64_t B,
+                                        int64_t M, int64_t N, int64_t H, int64_t W, void* stream);
 
 #ifdef __cplusplus
 }
